@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W              # configs[1] + configs[3]: the headline line
     python bench.py --config c3|c4|c5 ...                      # the other BASELINE configurations (one JSON line each)
     python bench.py --impl reference --gpus N ...              # the reference's CPU path (oracle port), rank 0 only
+    python bench.py ... --dump-outputs DIR                     # also write the last timed step's outputs as DIR/<name>.npy
 
 Default (config c2): a "step" = one pass of the extraction path over one batch: ResNet101-GeM descriptors of 64
 synthetic 1024x1024 RGB images per GPU (random-init weights of that architecture, inputs resident in HBM).  `value` is
@@ -19,6 +20,8 @@ roofline.search.
   c4: the search half alone (1000 x 1M, sharded).
   c5: multi-scale extraction (scales 0.7 / 1.0 / 1.4 of 1024^2, resized on the GPU) and alpha-QE (k=2, alpha=0.5)
       search on the sharded 1M database.
+Every GPU measurement on the line times --steps steps.  The inputs (images, weights, databases, queries) come from fixed
+seeds, so two builds run with the same arguments can be compared output for output with --dump-outputs.
 Prints ONE JSON line.
 """
 import argparse
@@ -59,7 +62,13 @@ def parse():
     ap.add_argument("--host-chunk", type=int, default=0)
     ap.add_argument("--search-n", type=int, default=SEARCH_N)
     ap.add_argument("--search-q", type=int, default=SEARCH_Q)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what each timed path returned in its last step as DIR/<name>.npy "
+                         "(float32 / float64, rank 0, at most 64 MB in all: larger outputs are cut to a seeded row sample)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    return args
 
 
 class ClockSampler(threading.Thread):
@@ -236,6 +245,7 @@ class Ctx:
         self.local = int(os.environ.get("LOCAL_RANK", "0"))
         torch.cuda.set_device(self.local)
         self.dist = None
+        self.last = None
         if self.world > 1:
             import torch.distributed as dist
             dist.init_process_group("nccl", device_id=torch.device("cuda", self.local))
@@ -268,24 +278,53 @@ class Ctx:
         return float(t.item())
 
     def timed(self, fn, steps):
-        """K calls of fn bracketed by barrier + synchronize, CUDA events on the current stream, max over ranks -> ms/step."""
+        """K calls of fn bracketed by barrier + synchronize, CUDA events on the current stream, max over ranks -> ms/step.
+        What the last call returned is left in self.last."""
         torch = self.torch
         self.barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            self.last = fn()
         e1.record()
         self.barrier()
         return self.max_over_ranks(e0.elapsed_time(e1)) / steps
 
     def wall(self, fn, steps):
+        """As timed(), on the host clock -> s/step."""
         self.barrier()
         t0 = time.perf_counter()
         for _ in range(steps):
-            fn()
+            self.last = fn()
         self.barrier()
         return self.max_over_ranks(time.perf_counter() - t0) / steps
+
+
+DUMP_BYTES = 64_000_000
+
+
+def keep(dump, name, value):
+    """Record an output of a timed path for --dump-outputs (dump is None when it was not asked for)."""
+    if dump is not None:
+        dump[name] = value
+
+
+def write_outputs(path, arrays):
+    """{name: tensor or array} -> path/<name>.npy: float64 for float64 and integer data (indices are exact below 2^53),
+    float32 otherwise.  An array over its share of DUMP_BYTES keeps a fixed, seeded sample of its rows, taken on the
+    device before the copy."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    budget = DUMP_BYTES // max(1, len(arrays)) - 4096          # 4 KB per file for the .npy header
+    for name, a in arrays.items():
+        a = torch.as_tensor(a)
+        a = a.double() if a.dtype == torch.float64 or not a.is_floating_point() else a.float()
+        if a.numel() * a.element_size() > budget:
+            rows = budget // (a[0].numel() * a.element_size())
+            pick = np.sort(np.random.RandomState(0).choice(a.shape[0], rows, replace=False))
+            a = a[torch.from_numpy(pick).to(a.device)]
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
 
 
 def make_net(args, ctx):
@@ -357,7 +396,7 @@ def conv_roofline(net, ctx, steps, fwd):
     return roof, layer_table, region_ms
 
 
-def bench_extract(args, ctx, line):
+def bench_extract(args, ctx, line, dump=None):
     import torch
     import synthdata as synth
     from dirb200 import ops
@@ -382,6 +421,8 @@ def bench_extract(args, ctx, line):
     ms_per_step = ctx.timed(lambda: net.forward(imgs, want_f16=True), args.steps)
     clocks = sampler.finish()
     value = world * B / (ms_per_step * 1e-3)
+    keep(dump, "descriptors", ctx.last[0])
+    keep(dump, "descriptors_f16", ctx.last[1])
 
     # ---- roofline from launches timed inside a sustained region of the same K steps
     roof, layer_table, region_ms = conv_roofline(net, ctx, args.steps, lambda: net.forward(imgs, want_f16=True))
@@ -401,13 +442,16 @@ def bench_extract(args, ctx, line):
     # ---- end to end through the C-ABI host entry point: pinned host images in, host descriptors out
     host = torch.empty((B, 3, S, S), dtype=torch.float32).pin_memory()
     host.copy_(imgs)
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     net.forward_host(host.numpy(), device=local)
     e2e_s = ctx.wall(lambda: net.forward_host(host.numpy(), device=local), e2e_steps)
     e2e_value = world * B / e2e_s
-    host8 = torch.randint(0, 256, (B, S, S, 3), dtype=torch.uint8).pin_memory()
+    keep(dump, "e2e_descriptors", ctx.last)
+    host8 = torch.randint(0, 256, (B, S, S, 3), generator=torch.Generator().manual_seed(1234 + rank),
+                          dtype=torch.uint8).pin_memory()
     net.forward_host_u8(host8.numpy(), device=local)
     e2e_u8 = world * B / ctx.wall(lambda: net.forward_host_u8(host8.numpy(), device=local), e2e_steps)
+    keep(dump, "e2e_u8_descriptors", ctx.last)
     del host8, host
 
     line.update({
@@ -435,7 +479,7 @@ def bench_extract(args, ctx, line):
                 net.forward(x)
             torch.cuda.synchronize()
             t0 = time.perf_counter()
-            n_it = 10
+            n_it = args.steps
             for _ in range(n_it):
                 net.forward(x)
             torch.cuda.synchronize()
@@ -456,9 +500,10 @@ def make_db(ctx, n_rows, d, seed=99):
     return db, db16, s0, s1
 
 
-def bench_search(args, ctx, n_rows, n_q, aqe=False, whiten=False, steps=None):
+def bench_search(args, ctx, n_rows, n_q, aqe=False, whiten=False, dump=None, name="search"):
     """queries/s of the exact top-k search on the row-sharded database (optionally: PCA-whitening of the queries first,
-    alpha query expansion = search + expand + search)."""
+    alpha query expansion = search + expand + search).  The last timed step's scores and indices go to dump as
+    <name>_scores / <name>_indices."""
     import torch
     import synthdata as synth
     from dirb200 import ops
@@ -490,9 +535,11 @@ def bench_search(args, ctx, n_rows, n_q, aqe=False, whiten=False, steps=None):
     for _ in range(3):
         step()
     index.check()
-    ssteps = steps or max(3, args.steps)
+    ssteps = args.steps
     s_ms = ctx.timed(step, ssteps)
     index.check()
+    keep(dump, name + "_scores", ctx.last[0])
+    keep(dump, name + "_indices", ctx.last[1])
     # phase profile of one more search (CUDA events inside the library, same stream)
     index.local.set_option("profile", 1)
     step()
@@ -543,7 +590,7 @@ def bench_search(args, ctx, n_rows, n_q, aqe=False, whiten=False, steps=None):
     return out, db, index
 
 
-def bench_whiten_block(ctx, db, D):
+def bench_whiten_block(ctx, db, D, steps, dump=None):
     import torch
     from dirb200 import ops
     gen = torch.Generator(device="cuda").manual_seed(5)
@@ -557,11 +604,12 @@ def bench_whiten_block(ctx, db, D):
     torch.cuda.synchronize()
     w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     w0.record()
-    for _ in range(3):
-        ops.whiten(x, comp, wmean, wcs)
+    for _ in range(steps):
+        y = ops.whiten(x, comp, wmean, wcs)
     w1.record()
     torch.cuda.synchronize()
-    w_ms = w0.elapsed_time(w1) / 3
+    w_ms = w0.elapsed_time(w1) / steps
+    keep(dump, "whiten", y)
     return {"rows": wn, "ms": w_ms, "rows_per_s": wn / (w_ms * 1e-3), "tflops_algorithmic": 2.0 * wn * D * D / (w_ms * 1e-3) / 1e12,
             "note": "x-mean -> prescaled fp16 hi/lo split, 3 tcgen05 GEMM passes, column scale, row L2 (<= 2e-5 vs fp64)"}
 
@@ -577,16 +625,17 @@ def main():
     world, rank = ctx.world, ctx.rank
     line = {"metric": None, "value": None, "unit": None, "n_gpus": world, "steps": args.steps, "warmup": max(3, args.warmup),
             "ms_per_step": None, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": None, "data": "synthetic"}
+    dump = {} if args.dump_outputs and rank == 0 else None
 
     if args.config == "c2":
-        net, imgs = bench_extract(args, ctx, line)
+        net, imgs = bench_extract(args, ctx, line, dump)
         if not args.no_search:
             del imgs
             net._release()
             torch.cuda.empty_cache()
-            s, db, index = bench_search(args, ctx, args.search_n, args.search_q)
+            s, db, index = bench_search(args, ctx, args.search_n, args.search_q, dump=dump)
             s["metric"] = "1M-DB queries/sec"
-            s["whiten"] = bench_whiten_block(ctx, db, SEARCH_D)
+            s["whiten"] = bench_whiten_block(ctx, db, SEARCH_D, args.steps, dump)
             line["search"] = s
             line["roofline"]["search"] = {"metric": s["metric"], "value": s["value"], "unit": s["unit"], "ms_per_step": s["ms_per_step"],
                                           "e2e": s["e2e"]["value"], "bound": s["roofline"]["bound"], "achieved": s["roofline"]["achieved"],
@@ -597,13 +646,13 @@ def main():
             index.disable_peer_exchange()
             del s, db, index
             torch.cuda.empty_cache()
-            sa, db, index = bench_search(args, ctx, args.search_n, args.search_q, aqe=True, steps=max(10, args.steps // 2))
+            sa, db, index = bench_search(args, ctx, args.search_n, args.search_q, aqe=True, dump=dump, name="search_aqe")
             line["roofline"]["search_aqe_c5"] = {"metric": "1M-DB alpha-QE queries/sec", "value": sa["value"], "unit": sa["unit"],
                                                  "ms_per_step": sa["ms_per_step"], "e2e": sa["e2e"]["value"], "config": sa["config"]}
             index.disable_peer_exchange()
             del sa, db, index
             torch.cuda.empty_cache()
-            s3, db, index = bench_search(args, ctx, C3_N * world, C3_Q, whiten=True, steps=max(20, args.steps))
+            s3, db, index = bench_search(args, ctx, C3_N * world, C3_Q, whiten=True, dump=dump, name="search_c3")
             line["roofline"]["search_c3"] = {"metric": "queries/sec, 70 x 100k per GPU + whitening", "value": s3["value"], "unit": s3["unit"],
                                              "ms_per_step": s3["ms_per_step"], "e2e": s3["e2e"]["value"], "bound": s3["roofline"]["bound"],
                                              "achieved": s3["roofline"]["achieved"], "peak": s3["roofline"]["peak"], "unit_roofline": s3["roofline"]["unit"],
@@ -615,10 +664,10 @@ def main():
         sampler = ClockSampler(ctx.local)
         sampler.start()
         if args.config == "c3":
-            s, db, index = bench_search(args, ctx, C3_N * world, C3_Q, whiten=True, steps=max(20, args.steps))
+            s, db, index = bench_search(args, ctx, C3_N * world, C3_Q, whiten=True, dump=dump)
             line["scaling"] = "weak"
         else:
-            s, db, index = bench_search(args, ctx, args.search_n, args.search_q)
+            s, db, index = bench_search(args, ctx, args.search_n, args.search_q, dump=dump)
             line["scaling"] = "strong"
         clocks = sampler.finish()
         line.update({"metric": "queries/sec", "value": s["value"], "unit": "queries/s", "ms_per_step": s["ms_per_step"], "steps": s["steps"],
@@ -642,7 +691,8 @@ def main():
         sampler.start()
         ms = ctx.timed(fwd, args.steps)
         clocks = sampler.finish()
-        roof, layer_table, _ = conv_roofline(net, ctx, max(1, min(args.steps, 3)), fwd)
+        keep(dump, "descriptors", ctx.last)
+        roof, layer_table, _ = conv_roofline(net, ctx, args.steps, fwd)
         host8 = u8.cpu().pin_memory()
 
         def e2e():
@@ -652,7 +702,8 @@ def main():
             out = net_.forward_u8_multiscale(h8.cuda(non_blocking=True), scales=(0.7, 1.0, 1.4), pooling="gem", gemp=3)
             return out.cpu()
         e2e()
-        e2e_s = ctx.wall(e2e, max(1, min(args.steps, 3)))
+        e2e_s = ctx.wall(e2e, args.steps)
+        keep(dump, "e2e_descriptors", ctx.last)
         flops_img = (161.81 + 325.99 + 644.21) * (S / 1024.0) ** 2 * 1e9        # SURVEY 8d: R101 at 717 / 1024 / 1434
         line.update({"metric": "multi-scale descriptor images/sec", "value": world * B / (ms * 1e-3), "unit": "images/s", "ms_per_step": ms,
                      "dtype": "f16 operands, f32 accumulate",
@@ -666,7 +717,7 @@ def main():
         del u8
         net._release()
         torch.cuda.empty_cache()
-        s, db, index = bench_search(args, ctx, args.search_n, args.search_q, aqe=True)
+        s, db, index = bench_search(args, ctx, args.search_n, args.search_q, aqe=True, dump=dump, name="search_aqe")
         s["metric"] = "1M-DB alpha-QE queries/sec"
         line["search"] = s
         line["roofline"]["search"] = {"metric": s["metric"], "value": s["value"], "unit": s["unit"], "ms_per_step": s["ms_per_step"],
@@ -692,6 +743,8 @@ def main():
                                                "" if n == full_n else ", scaled to %d rows" % full_n)}
     if rank == 0:
         print(json.dumps(line))
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if "index" in locals():
         locals()["index"].disable_peer_exchange()      # unmap the peers' windows before any rank frees its own
     if ctx.dist is not None:
