@@ -1336,16 +1336,28 @@ int dirb200_index_rank_count(dirb200_index* h, const float* q32, int Q, const in
   return 0;
 }
 
+// merge_lists_kernel holds all G*k (fp64 score, int64 index) entries of a query in dynamic shared memory: up to
+// MERGE_MAX_ENTRIES * 16 = 64 KiB.  Without opting in a launch gets 48 KiB including the kernel's static shared memory,
+// so G*k >= 3072 would fail to launch.
+constexpr int MERGE_MAX_ENTRIES = 4096;
+static int merge_smem_opt_in() {
+  static std::atomic<uint64_t> attr_done{0};
+  if (first_launch_on_device(attr_done))
+    DIRB_CUDA(cudaFuncSetAttribute(merge_lists_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, MERGE_MAX_ENTRIES * 16));
+  return 0;
+}
+
 int dirb200_topk_merge(const double* scores_dev, const int64_t* idx_dev, int G, int Q, int k, int64_t shard_stride,
                        double* out_scores_dev, int64_t* out_idx_dev, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DIRB_REQUIRE(scores_dev && idx_dev && out_scores_dev && out_idx_dev, DIRB200_EINVAL, "null argument");
-  DIRB_REQUIRE(G >= 1 && Q >= 1 && k >= 1 && static_cast<int64_t>(G) * k <= 4096, DIRB200_ENOTSUP,
-               "merge supports G*k <= 4096 (got G=%d k=%d)", G, k);
+  DIRB_REQUIRE(G >= 1 && Q >= 1 && k >= 1 && static_cast<int64_t>(G) * k <= MERGE_MAX_ENTRIES, DIRB200_ENOTSUP,
+               "merge supports G*k <= %d (got G=%d k=%d)", MERGE_MAX_ENTRIES, G, k);
   // shard g holds [Q][k] at element offset g*shard_stride, each list already ordered: rank-based merge, read in place
   if (shard_stride <= 0) shard_stride = static_cast<int64_t>(Q) * k;
   const int n = G * k;
   const int threads = std::min(1024, (n + 31) / 32 * 32);
+  DIRB_TRY(merge_smem_opt_in());
   merge_lists_kernel<<<Q, threads, static_cast<size_t>(n) * 16, stream>>>(scores_dev, idx_dev, G, k, shard_stride, out_scores_dev,
                                                                         out_idx_dev, PeerX{}, nullptr);
   count_launch();
@@ -1378,8 +1390,8 @@ int dirb200_exchange_create(int device, int world, int rank, int max_q, int max_
   DIRB_REQUIRE(out, DIRB200_EINVAL, "null argument");
   DIRB_REQUIRE(world >= 1 && world <= X_MAXW && rank >= 0 && rank < world, DIRB200_ENOTSUP,
                "peer exchange supports 1..%d ranks of one box (got world=%d rank=%d)", X_MAXW, world, rank);
-  DIRB_REQUIRE(max_q >= 1 && max_k >= 1 && max_k <= 1024 && static_cast<int64_t>(world) * max_k <= 4096, DIRB200_ENOTSUP,
-               "need max_q >= 1, 1 <= max_k <= 1024 and world * max_k <= 4096");
+  DIRB_REQUIRE(max_q >= 1 && max_k >= 1 && max_k <= 1024 && static_cast<int64_t>(world) * max_k <= MERGE_MAX_ENTRIES,
+               DIRB200_ENOTSUP, "need max_q >= 1, 1 <= max_k <= 1024 and world * max_k <= %d", MERGE_MAX_ENTRIES);
   DIRB_TRY(dirb200_device_check(device));
   DIRB_CUDA(cudaSetDevice(device));
   auto* x = new dirb200_exchange();
@@ -1518,6 +1530,7 @@ int dirb200_index_search_sharded_phase(dirb200_index* h, dirb200_exchange* x, in
   DIRB_REQUIRE(phase == 4 && scores_dev && idx_dev, DIRB200_EINVAL, "phase is 1 .. 4 (4 needs the output buffers)");
   const int n = x->world * k;
   const int threads = std::min(1024, (n + 31) / 32 * 32);
+  DIRB_TRY(merge_smem_opt_in());
   merge_lists_kernel<<<Q, threads, static_cast<size_t>(n) * 16, stream>>>(nullptr, nullptr, x->world, k, 0, scores_dev, idx_dev, px,
                                                                         h->pend.status ? h->pend.status : x->status);
   count_launch();
