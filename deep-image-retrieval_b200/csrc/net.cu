@@ -932,14 +932,15 @@ int dirb200_net_profile_table(dirb200_net* n, char* buf, size_t cap, size_t* nee
 
 int dirb200_net_debug_stage(dirb200_net* n, const char* what, void* dst_dev, size_t capacity, int dims[4],
                             void* stream_) {
-  DIRB_REQUIRE(n && what && dst_dev && dims, DIRB200_EINVAL, "null argument");
+  DIRB_REQUIRE(n && what && dims, DIRB200_EINVAL, "null argument");
   auto it = n->taps.find(what);
   DIRB_REQUIRE(it != n->taps.end() && it->second.ptr, DIRB200_EKEY,
                "no stage '%s' recorded (set option debug_taps=1 and run a forward first)", what);
   const auto& t = it->second;
   const size_t bytes = static_cast<size_t>(t.n) * t.h * t.w * t.c * 2;
+  dims[0] = t.n; dims[1] = t.h; dims[2] = t.w; dims[3] = t.c;     // also when the buffer is too small: size query
+  if (!dst_dev) return 0;
   DIRB_REQUIRE(bytes <= capacity, DIRB200_EINVAL, "stage '%s' needs %zu bytes", what, bytes);
-  dims[0] = t.n; dims[1] = t.h; dims[2] = t.w; dims[3] = t.c;
   DIRB_CUDA(cudaMemcpyAsync(dst_dev, t.ptr, bytes, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream_)));
   return 0;
 }

@@ -315,14 +315,16 @@ class ResNetRMAC:
         return h
 
     def debug_stage(self, what):
-        """NHWC fp16 activation after 'stem' / 'layer1'..'layer4' of the last chunk of the last forward."""
+        """NHWC fp16 activation after 'stem' / 'layer1'..'layer4' ('fpn_c4': the merged layer3 map of an FPN head) of
+        the last chunk of the last forward (needs set_backend_option('debug_taps', 1))."""
         dims = (C.c_int * 4)()
-        dev = torch.device("cuda", self._handle_device)
-        buf = torch.empty(1 << 28, dtype=torch.uint8, device=dev)
-        lib.call("dirb200_net_debug_stage", self._handle, what.encode(), C.c_void_p(buf.data_ptr()), buf.numel(), dims,
-                 C.c_void_p(torch.cuda.current_stream().cuda_stream))
+        stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+        lib.call("dirb200_net_debug_stage", self._handle, what.encode(), C.c_void_p(0), 0, dims, stream)   # size query
         n, hh, ww, c = [int(v) for v in dims]
-        return buf[: n * hh * ww * c * 2].view(torch.float16).view(n, hh, ww, c).clone()
+        out = torch.empty((n, hh, ww, c), dtype=torch.float16, device=torch.device("cuda", self._handle_device))
+        lib.call("dirb200_net_debug_stage", self._handle, what.encode(), C.c_void_p(out.data_ptr()), out.numel() * 2, dims,
+                 stream)
+        return out
 
     def profile(self):
         """Per-class timing of the last forward (needs set_backend_option('profile', 1)):

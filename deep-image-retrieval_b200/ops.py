@@ -142,6 +142,14 @@ def maxpool_3x3s2(x):
     return out
 
 
+def center_bias(x, b):
+    """In place on x (NHWC fp16 (B,H,W,C)): x *= 1 + the center-bias map of rmac_resnet.py:52-56; returns x."""
+    _chk(x, torch.float16, "x")
+    bb, h, w, c = x.shape
+    lib.call("dirb200_center_bias", _ptr(x), bb, h, w, c, float(b), _stream())
+    return x
+
+
 POOLING = {"gem": 0, "max": 1, "avg": 2}
 
 

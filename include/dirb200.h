@@ -60,7 +60,9 @@ int dirb200_device_check(int device);
  * dirb200_net_set_option forwards these keys here. */
 int dirb200_set_global_option(const char* key, double value);
 int dirb200_get_global_option(const char* key, double* value);
-/* arch: "resnet50_rmac" | "resnet101_rmac" | "resnet152_rmac" (Bottleneck trunks, rmac_resnet.py:78-88). */
+/* arch: "resnet18_rmac" (BasicBlock trunk) | "resnet50_rmac" | "resnet101_rmac" | "resnet152_rmac" (Bottleneck trunks,
+ * rmac_resnet.py:74-88), or the FPN heads "resnet{18,50,101,152}_fpn_rmac" (mode 1) and "resnet101_fpn0_rmac" (mode 0,
+ * rmac_resnet_fpn.py:92-110). */
 int dirb200_net_create(const char* arch, int device, dirb200_net** out);
 /* Options.
  * Model options of rmac_resnet.py:15-37 (the three marked * must be set BEFORE dirb200_net_finalize, later
@@ -72,8 +74,10 @@ int dirb200_net_create(const char* arch, int device, dirb200_net** out);
  * images per sub-chunk of stem / layer1..4), 0 (default, faster as measured) = whole chunk per stage.
  * Implementation A/B switches: "conv_impl" 0 = persistent tcgen05 implicit GEMM (default), 1 = mma.sync implicit
  * GEMM (validation path), 2 = one-tile-per-CTA tcgen05 kernel (baseline); "fuse_ds" 1 (default) = projection
- * shortcut fused into conv3 as a K-concatenated GEMM; "fuse_c23" 1 (default) = conv2 + conv3 (+ residual) of the
- * identity blocks with 64 / 128 / 256 mid channels as one kernel (dirb200_conv_c23).  PROCESS-WIDE (they select kernels, not handle state; set
+ * shortcut fused into conv3 as a K-concatenated GEMM; "fuse_c23" 0 (default, the fused kernel measured slower,
+ * DESIGN.md section 7) / 1 where every SM gets several tiles / 2 wherever the kernel supports the shape = conv2 + conv3
+ * (+ residual) of the identity blocks with 64 / 128 / 256 mid channels as one kernel (dirb200_conv_c23), "c23_variant"
+ * 1 (default) = CTA pairs, 0 = one CTA per tile.  PROCESS-WIDE (they select kernels, not handle state; set
  * them once, not concurrently with a running forward): "halo" 1 (default) / 0 = 3x3 stride-1 convolutions load
  * their input patch once per tile (conv_halo.cuh) or tap by tap; "pdl" 1 (default) = programmatic dependent
  * launch between consecutive kernels; "res_variant" tile-variant selector of the residual 1x1 convolutions.
@@ -109,8 +113,11 @@ int dirb200_net_forward_host_u8(dirb200_net* net, const uint8_t* imgs_host, int 
  * call with kk_out == NULL to query ksize). */
 int dirb200_resize_bilinear_u8(const uint8_t* in_dev, int B, int H, int W, int Ho, int Wo, uint8_t* out_dev, void* stream);
 int dirb200_resize_coeffs(int in_size, int out_size, int* bounds_out, int* kk_out, int* ksize_out);
-/* Debug tap (needs option "debug_taps"): copy the NHWC fp16 activation after stage `what` ("stem","layer1".."layer4")
- * of the LAST chunk of the last forward into dst_dev (capacity in bytes); returns its dims as {n,h,w,c}. */
+/* Debug tap (needs option "debug_taps"): copy the NHWC fp16 activation after stage `what` ("stem","layer1".."layer4",
+ * "fpn_c4" for FPN heads of mode 1) of the LAST chunk of the last forward into dst_dev (capacity in bytes); returns
+ * its dims as {n,h,w,c}.  "layer4" and "fpn_c4" hold the last sub-chunk of that chunk (option "stage_sched").
+ * Two-call protocol: dst_dev = NULL only fills dims; dims are filled as well when capacity is too small
+ * (DIRB200_EINVAL), so the caller can size its buffer as n*h*w*c*2 bytes. */
 int dirb200_net_debug_stage(dirb200_net* net, const char* what, void* dst_dev, size_t capacity, int dims[4],
                             void* stream);
 /* Per-class CUDA-event timing of the last forward run with option "profile" = 1: out16 = 4 rows of

@@ -80,11 +80,13 @@ def test_conv_bn_act(case, impl):
     assert err <= tol, (err, tol)
 
 
-@pytest.mark.parametrize("knobs", [dict(epi_mode=0), dict(epi_mode=1), dict(epi_mode=2), dict(epi_mode=3),
-                                   dict(epi_mode=3, l2_prefetch=1), dict(epi_mode=2, res_variant=1), dict(epi_mode=3, res_variant=2),
-                                   dict(epi_mode=3, res_variant=3, l2_prefetch=8), dict(epi_mode=0, res_variant=3),
-                                   dict(epi_warps=8), dict(epi_warps=16), dict(epi_warps=16, epi_mode=2), dict(epi_warps=8, epi_mode=1)],
-                         ids=lambda k: ",".join("%s=%d" % kv for kv in k.items()))
+EPI_KNOBS = [dict(epi_mode=0), dict(epi_mode=1), dict(epi_mode=2), dict(epi_mode=3),
+             dict(epi_mode=3, l2_prefetch=1), dict(epi_mode=2, res_variant=1), dict(epi_mode=3, res_variant=2),
+             dict(epi_mode=3, res_variant=3, l2_prefetch=8), dict(epi_mode=0, res_variant=3),
+             dict(epi_warps=8), dict(epi_warps=16), dict(epi_warps=16, epi_mode=2), dict(epi_warps=8, epi_mode=1)]
+
+
+@pytest.mark.parametrize("knobs", EPI_KNOBS, ids=lambda k: ",".join("%s=%d" % kv for kv in k.items()))
 def test_conv_epilogue_and_tile_variants(knobs):
     """Every epilogue organisation (one / two warp groups, late / early release of the residual staging buffers), residual
     tile variant and the next-tile L2 prefetch compute the same convolution: the residual and many-tile cases of
@@ -220,8 +222,11 @@ def test_conv_c23_fused_bottleneck_tail(cm, b, h, w, variant):
     """conv2 (3x3) + BN + ReLU + conv3 (1x1) + BN + residual + ReLU in ONE kernel (resnet.py:75-85) == the two-kernel
     path bit for bit (same fp16 rounding of the intermediate, same K order), and within fp16 tolerance of the oracle;
     ragged tiles (sizes that are not multiples of the 8 x 16 patch) and many tiles per CTA."""
-    ops = _ops()
-    r = np.random.RandomState(cm + h)
+    _conv_c23_case(_ops(), cm, b, h, w, variant, seed=cm + h)
+
+
+def _conv_c23_case(ops, cm, b, h, w, variant, seed):
+    r = np.random.RandomState(seed)
     t1 = torch.from_numpy(np.maximum(r.standard_normal((b, h, w, cm)), 0).astype(np.float16)).to(DEV)
     res = torch.from_numpy(r.standard_normal((b, h, w, 4 * cm)).astype(np.float16)).to(DEV)
     w2 = torch.from_numpy((r.standard_normal((cm, cm, 3, 3)) * np.sqrt(2.0 / (9 * cm))).astype(np.float32))
